@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — upscaled Mpixels/s of the FSR 1.0 hot path (EASU+RCAS) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one synthetic frame through EASU -> RCAS.  Default workload = BASELINE.json configs[1]:
 1920x1080 -> 3840x2160, RGBA16F, sharpness 0.25 stops.  With N > 1 (launched by torchrun, one rank per GPU)
@@ -41,6 +41,7 @@ WORKLOADS = {
 SHARPNESS = 0.25
 RING = 8
 METRIC = "upscaled Mpixels/sec (EASU+RCAS)"
+DUMP_PIXELS = 1 << 21                  # --dump-outputs: at most 2M RGBA float32 pixels (32 MB) over all ranks
 
 
 def load_peaks():
@@ -431,6 +432,10 @@ def run_ours(args, rank, world, local_rank):
     launches = api.launch_count() - launches0
     clocks = (sampler.stop() if not os.environ.get("FSR1_BENCH_NO_SAMPLER") else sampler._smi_once()) if rank == 0 else None
     up.status()
+    if args.dump_outputs:
+        # the slot of the last timed step; the nccl step numbers frames on from the warm-up
+        last = (K - 1) % RING if halo_mode == "p2p" else (frame_no[0] - 1) % RING
+        dump_output(args.dump_outputs, "output" if world == 1 else "output_rank%d" % rank, up.output(last), DUMP_PIXELS // world)
     if args.trace and world > 1 and halo_mode == "p2p":
         tr = up.trace().astype(np.int64)
         os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
@@ -628,6 +633,20 @@ def run_ours(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+def dump_output(dirname, name, out, max_pixels):
+    """Writes dirname/name.npy: the [rows, width, 4] image `out` as float32 [n, 4], the pixels in row-major order; above
+    max_pixels a fixed sample of them (numpy default_rng(0)), so that two builds write the same pixels."""
+    import numpy as np
+    import torch
+    rows, width = out.shape[:2]
+    n = rows * width
+    idx = np.arange(n) if n <= max_pixels else np.sort(np.random.default_rng(0).choice(n, max_pixels, replace=False))
+    idx = torch.from_numpy(idx).to(out.device)
+    pix = out[idx // width, idx % width].float().cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), pix)
+
+
 def check_sharded_parity(F, api, up, dist, dev, rank, world, iw, ih, ow, oh, H_in, H_out, tdt, rank_rows, halo_mode):
     """Outside the timed region: frame 0 once more through the sharded path, every rank's slab sent to rank 0, which upscales the
     whole frame on its own GPU and compares bit for bit; then against the oracle on bands that straddle slab boundaries; then
@@ -723,7 +742,14 @@ def main():
     ap.add_argument("--fused", action="store_true", help="FSR1_FLAG_FUSED: EASU and RCAS in one kernel (intermediate in shared memory); roofline against bpp*(Pin+Pout)")
     ap.add_argument("--trace", action="store_true", help="multi-GPU p2p: print device-timestamp statistics of the halo hand-shake per rank (stderr)")
     ap.add_argument("--halo", default="p2p", choices=["p2p", "nccl"], help="multi-GPU halo data plane: direct NVLink stores through the C ABI (default) or NCCL send/recv")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the upscaled frame of the last one as DIR/output.npy "
+                    "(DIR/output_rank<r>.npy per rank with --gpus > 1): float32 [n, 4] RGBA pixels, a fixed seeded sample of 2M "
+                    "pixels of a larger frame; the inputs are the same every run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,18 +1,18 @@
 #!/usr/bin/env bash
 # TEST INFRASTRUCTURE — builds oracle/_ref/libfsr1_ref.so from the reference's own sources where
-# they lie under /root/reference (SURVEY.md §8(c), Appendix A).  Nothing from the reference is
-# copied into the repo: the rewritten headers live in a mktemp directory that is deleted, and the
-# only output is the shared library under oracle/_ref/ (git-ignored, travels with gpurun).
+# FSR1_REFERENCE_DIR names a checkout of GPUOpen-Effects/FidelityFX-FSR (SURVEY.md §8(c), Appendix A).
+# Nothing from the reference is copied into the repo: the rewritten headers live in a mktemp directory
+# that is deleted, and the only output is the shared library under oracle/_ref/ (git-ignored).
 #
 # The rewrite is purely mechanical (HLSL parameter qualifiers -> C++):
 #   inout AXn name -> AXn& name ; out AXn name -> AXn& name ; in AXn name -> AXn name
 #   and the three AZolZeroPassF{2,3,4} helpers (vector ?: — inexpressible in C++, unused by FSR1) removed.
 set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
-REF="${FSR1_REFERENCE_DIR:-/root/reference}/ffx-fsr"
+REF="${FSR1_REFERENCE_DIR:-}/ffx-fsr"
 OUT="$HERE/_ref"
-if [ ! -f "$REF/ffx_fsr1.h" ]; then
-  echo "build_ref: $REF not present (GPU box?) — keeping prebuilt $OUT" >&2
+if [ -z "${FSR1_REFERENCE_DIR:-}" ] || [ ! -f "$REF/ffx_fsr1.h" ]; then
+  echo "build_ref: FSR1_REFERENCE_DIR does not name a reference checkout — keeping $OUT as it is (without it the tests compare with the stored digests only)" >&2
   exit 0
 fi
 mkdir -p "$OUT"

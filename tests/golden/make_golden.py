@@ -1,6 +1,6 @@
 """Generates tests/golden/*.npz and kat.json by EXECUTING THE REFERENCE (oracle/_ref/libfsr1_ref.so =
-the reference's own ffx_fsr1.h source compiled for the host, see oracle/build_ref.sh).  Run in the
-build container (needs /root/reference); the outputs are committed so the GPU box can use them.
+the reference's own ffx_fsr1.h source compiled for the host, see oracle/build_ref.sh).  Needs
+FSR1_REFERENCE_DIR; the outputs are committed so the tests run where the reference is absent.
 
     python tests/golden/make_golden.py
 """
@@ -17,7 +17,7 @@ import oracle_lib as ol  # noqa: E402
 import fsr1_b200 as F  # noqa: E402
 
 R = ol.ref()
-assert R is not None, "reference build missing: run oracle/build_ref.sh where /root/reference exists"
+assert R is not None, "reference build missing: set FSR1_REFERENCE_DIR to a checkout of the reference and run oracle/build_ref.sh"
 
 IW, IH = 32, 18
 SIZES = {"x2.0": (64, 36), "x1.5": (48, 27), "x1.3": (41, 23), "x1.0": (32, 18), "x2.0x1.5": (64, 27)}

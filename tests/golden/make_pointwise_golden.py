@@ -1,6 +1,6 @@
 """Generates tests/golden/fsr1_pointwise_golden.npz by EXECUTING THE REFERENCE's own FsrSrtmF / FsrSrtmInvF / FsrLfgaF /
-FsrTepdDitF / FsrTepdC8F / FsrTepdC10F (oracle/_ref/libfsr1_ref.so, see oracle/build_ref.sh).  Run in the build
-container (needs /root/reference); the output is committed so the GPU box can use it.
+FsrTepdDitF / FsrTepdC8F / FsrTepdC10F (oracle/_ref/libfsr1_ref.so, see oracle/build_ref.sh).  Needs
+FSR1_REFERENCE_DIR; the output is committed so the tests run where the reference is absent.
 
     python tests/golden/make_pointwise_golden.py
 """
@@ -16,7 +16,7 @@ import oracle_lib as ol  # noqa: E402
 import fsr1_b200 as F  # noqa: E402
 
 R = ol.ref()
-assert R is not None, "reference build missing: run oracle/build_ref.sh where /root/reference exists"
+assert R is not None, "reference build missing: set FSR1_REFERENCE_DIR to a checkout of the reference and run oracle/build_ref.sh"
 
 W, H = 300, 11                                  # wider than one 256-thread CTA row, no multiple of any tile size
 fix = {}

@@ -1,8 +1,8 @@
 """Generates tests/golden/fsr1_pointwise_h_golden.npz by EXECUTING THE REFERENCE's own half-precision functions FsrSrtmH /
 FsrSrtmInvH / FsrLfgaH / FsrTepdDitH / FsrTepdC8H / FsrTepdC10H and their packed Hx2 forms, plus FsrRcasHx2 with the
 compile-time options (oracle/_ref/libfsr1_ref.so built with A_HALF, see oracle/build_ref.sh).  The H and the Hx2 results are
-asserted bit-identical before one copy is stored.  Run in the build container (needs /root/reference); the output is committed
-so the checks also run where the reference build is absent.
+asserted bit-identical before one copy is stored.  Needs FSR1_REFERENCE_DIR; the output is committed so the
+checks also run where the reference build is absent.
 
     python tests/golden/make_pointwise_h_golden.py
 """
@@ -18,7 +18,7 @@ import oracle_lib as ol  # noqa: E402
 import fsr1_b200 as F  # noqa: E402
 
 R = ol.ref()
-assert R is not None, "reference build missing: run oracle/build_ref.sh where /root/reference exists"
+assert R is not None, "reference build missing: set FSR1_REFERENCE_DIR to a checkout of the reference and run oracle/build_ref.sh"
 
 
 def u16(a):

@@ -1,6 +1,9 @@
 """ctypes access to the CPU oracle (oracle/libfsr1_oracle.so) and, when it was built, to the reference's
 own source compiled for the host (oracle/_ref/libfsr1_ref.so).  TEST INFRASTRUCTURE ONLY."""
+import atexit
 import ctypes
+import hashlib
+import json
 import os
 import subprocess
 
@@ -17,7 +20,8 @@ def build():
     if not os.path.exists(ORACLE_SO) or os.path.getmtime(ORACLE_SO) < os.path.getmtime(src):
         subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "libfsr1_oracle.so"],
                               stdout=subprocess.DEVNULL)
-    if not os.path.exists(REF_SO) and os.path.exists("/root/reference/ffx-fsr/ffx_fsr1.h"):
+    ref_dir = os.environ.get("FSR1_REFERENCE_DIR")
+    if not os.path.exists(REF_SO) and ref_dir and os.path.exists(os.path.join(ref_dir, "ffx-fsr", "ffx_fsr1.h")):
         subprocess.check_call([os.path.join(ROOT, "oracle", "build_ref.sh")], stdout=subprocess.DEVNULL)
 
 
@@ -45,6 +49,46 @@ def ref():
         _r.fsr1ref_cpu_f32_to_f16.restype = ctypes.c_uint32
         _r.fsr1ref_cpu_f32_to_f16.argtypes = [F]
     return _r
+
+
+DIGESTS = os.path.join(ROOT, "tests", "golden", "reference_digests.json")
+_digests, _recorded = None, {}
+
+
+def _record_at_exit():
+    with open(os.environ["FSR1_RECORD_DIGESTS"], "w") as f:
+        json.dump(dict(sorted(_recorded.items())), f, indent=0)
+
+
+if os.environ.get("FSR1_RECORD_DIGESTS"):
+    atexit.register(_record_at_exit)
+
+
+def pinned(key, got, *live):
+    """`got` (array-like) must be what the reference's own source computes for the inputs `key` names.  Where the reference build
+    exists, every live() is computed and compared bit for bit.  Always, the SHA-256 of got's bytes is compared with the one stored
+    for `key` in tests/golden/reference_digests.json, so the comparison also runs where the reference is absent.  Those digests were
+    recorded from the oracle (FSR1_RECORD_DIGESTS=<file> python -m pytest tests/test_oracle.py tests/test_constants.py
+    tests/test_emu_hx2.py), which these same tests hold bit-equal to the reference build wherever it is present."""
+    got = np.ascontiguousarray(got)
+    if ref() is not None:
+        for fn in live:
+            want = np.ascontiguousarray(fn())
+            assert want.shape == got.shape and want.tobytes() == got.tobytes(), key
+    d = hashlib.sha256(got.tobytes()).hexdigest()
+    if os.environ.get("FSR1_RECORD_DIGESTS"):
+        assert _recorded.setdefault(key, d) == d, key
+        return
+    global _digests
+    if _digests is None:
+        with open(DIGESTS) as f:
+            _digests = json.load(f)
+    assert _digests.get(key) == d, key
+
+
+def rcas_key(prec, gen, w, h, seed, sharp, clamp, denoise=False, alpha=False):
+    """The `pinned` key of an RCAS of frames.<gen>(w, h, seed) (prec "h16": quantised to half)."""
+    return "rcas_%s %s %dx%d seed%d s%g c%d dn%d pa%d" % (prec, gen, w, h, seed, sharp, clamp, denoise, alpha)
 
 
 def _con(n):

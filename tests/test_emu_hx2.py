@@ -61,9 +61,9 @@ def test_emulated_rcas_hx2_bit_identical_to_the_half_oracle(size, gen):
         for clamp in (False, True):
             got = emu_rcas_hx2(img, rc, clamp)
             assert np.array_equal(bits(got), bits(ol.rcas(img, rc, clamp)))
-            if R is not None and sharp == 0.25:
-                assert np.array_equal(bits(got), bits(ol.rcas_hx2(img, rc, clamp)))     # the reference's own FsrRcasHx2
-                assert np.array_equal(bits(got), bits(ol.rcas(img, rc, clamp, lib=R)))  # and its FsrRcasH
+            if sharp == 0.25:         # the reference's own FsrRcasHx2 and FsrRcasH, live or through their stored digests
+                ol.pinned(ol.rcas_key("h16", gen, w, h, 321, sharp, clamp), got,
+                          lambda: ol.rcas_hx2(img, rc, clamp), lambda: ol.rcas(img, rc, clamp, lib=R))
 
 
 @pytest.mark.parametrize("denoise,alpha", [(True, False), (False, True), (True, True)])
@@ -75,8 +75,8 @@ def test_emulated_rcas_hx2_options(denoise, alpha):
     for clamp in (False, True):
         got = emu_rcas_hx2(img, rc, clamp, opts=opts)
         assert np.array_equal(bits(got), bits(ol.rcas(img, rc, clamp, denoise=denoise, alpha=alpha)))
-        if ol.ref() is not None:
-            assert np.array_equal(bits(got), bits(ol.rcas_hx2(img, rc, clamp, denoise=denoise, alpha=alpha)))
+        ol.pinned(ol.rcas_key("h16", "structured", w, h, 77, 0.25, clamp, denoise, alpha), got,
+                  lambda: ol.rcas_hx2(img, rc, clamp, denoise=denoise, alpha=alpha))
         if alpha:
             assert np.array_equal(bits(got[..., 3]), bits(img[..., 3]))
 
@@ -109,37 +109,35 @@ def test_emulated_pointwise_hx2_bit_identical_to_the_half_oracle(size):
     w, h = size
     sdr, hdr, grain, noise = _frames(w, h)
     R = ol.ref()
-    libs = [None] + ([R] if R is not None else [])
+    k = "emu_frames %dx%d " % (w, h)      # the reference's H (and Hx2) functions: live or through their stored digests
     # SRTM and its inverse (incl. the c = 1.0 case the extra max solves)
     t = emu_point(1, hdr)
-    for lib in libs:
-        assert np.array_equal(bits(t), bits(ol.srtm_h(hdr, lib=lib)))
+    assert np.array_equal(bits(t), bits(ol.srtm_h(hdr)))
+    ol.pinned(k + "srtm", t, lambda: ol.srtm_h(hdr, lib=R), lambda: ol.srtm_h(hdr, lib=R, hx2=True))
     ti = emu_point(2, t)
     one = F.to_half(np.ones((2, 20, 4), np.float32))
-    for lib in libs:
-        assert np.array_equal(bits(ti), bits(ol.srtm_h(t, inverse=True, lib=lib)))
-        assert np.array_equal(bits(emu_point(2, one)), bits(ol.srtm_h(one, inverse=True, lib=lib)))
-    if R is not None:
-        assert np.array_equal(bits(t), bits(ol.srtm_h(hdr, lib=R, hx2=True)))
+    t1 = emu_point(2, one)
+    assert np.array_equal(bits(ti), bits(ol.srtm_h(t, inverse=True)))
+    assert np.array_equal(bits(t1), bits(ol.srtm_h(one, inverse=True)))
+    ol.pinned(k + "srtm_inv", ti, lambda: ol.srtm_h(t, inverse=True, lib=R))
+    ol.pinned("emu_frames ones 20x2 srtm_inv", t1, lambda: ol.srtm_h(one, inverse=True, lib=R))
     assert np.array_equal(bits(t[..., 3]), bits(hdr[..., 3]))      # alpha carried through
     # LFGA
     for amount in (0.0, 0.35, 1.0):
         got = emu_point(3, sdr, aux=grain, amount=amount)
-        for lib in libs:
-            assert np.array_equal(bits(got), bits(ol.lfga_h(sdr, grain, amount, lib=lib)))
-        if R is not None:
-            assert np.array_equal(bits(got), bits(ol.lfga_h(sdr, grain, amount, lib=R, hx2=True)))
+        assert np.array_equal(bits(got), bits(ol.lfga_h(sdr, grain, amount)))
+        ol.pinned(k + "lfga %g" % amount, got, lambda: ol.lfga_h(sdr, grain, amount, lib=R),
+                  lambda: ol.lfga_h(sdr, grain, amount, lib=R, hx2=True))
     # TEPD, positional dither (FsrTepdDitHx2: p and p + (8,0)) and a blue-noise tile
     for nbits, op in ((8, 4), (10, 5)):
         for frame in (0, 5):
             got = emu_point(op, sdr, frame=frame)
-            for lib in libs:
-                assert np.array_equal(bits(got), bits(ol.tepd_h(sdr, nbits, frame=frame, lib=lib)))
-            if R is not None:
-                assert np.array_equal(bits(got), bits(ol.tepd_h(sdr, nbits, frame=frame, lib=R, hx2=True)))
+            assert np.array_equal(bits(got), bits(ol.tepd_h(sdr, nbits, frame=frame)))
+            ol.pinned(k + "tepd%d f%d positional" % (nbits, frame), got, lambda: ol.tepd_h(sdr, nbits, frame=frame, lib=R),
+                      lambda: ol.tepd_h(sdr, nbits, frame=frame, lib=R, hx2=True))
         got = emu_point(op, sdr, aux=noise)
-        for lib in libs:
-            assert np.array_equal(bits(got), bits(ol.tepd_h(sdr, nbits, dither=noise, lib=lib)))
+        assert np.array_equal(bits(got), bits(ol.tepd_h(sdr, nbits, dither=noise)))
+        ol.pinned(k + "tepd%d noise" % nbits, got, lambda: ol.tepd_h(sdr, nbits, dither=noise, lib=R))
 
 
 def test_emulated_pointwise_hx2_row_range_in_place_semantics():
