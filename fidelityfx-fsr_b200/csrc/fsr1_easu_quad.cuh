@@ -21,16 +21,17 @@ __device__ __forceinline__ float texel_luma(uint2 t) {  // 2*luma = 0.5 B + (0.5
   return fmaf(__low2float(u2h2(t.y)), 0.5f, fmaf(rg.x, 0.5f, rg.y));
 }
 
-// Window weight of two pixels at squared distance d2: ((d2/4 - 5/4) d2 + 1)(lob d2 - 1)^2, the Horner form of
-// (25/16 (2/5 d2 - 1)^2 - 9/16)(lob d2 - 1)^2 (ffx_fsr1.h:255-270).  The clamp min(d2, clp) is a packed 16-bit INTEGER
-// min (VIMNMX.S16x2, integer pipe): clp > 0, so comparing the bit patterns as signed integers orders every
-// non-negative d2 correctly and returns d2 itself when rounding made it slightly negative — identical to __hmin2 for
-// finite inputs, off the pipe the HFMA2s use.
+// Window weight of two pixels at squared distance d2, times 4: (25/16 (2/5 d2 - 1)^2 - 9/16)(lob d2 - 1)^2
+// (ffx_fsr1.h:255-270) = (d2 - 1)(d2 - 4)(lob d2 - 1)^2 / 4.  With v = lob d2 - 1 and p = (d2 - 1) v the product is
+// p (p - 3 v): four HFMA2/HMUL2 instead of five, and no rounded sum of large terms (each factor is one FMA of the exact
+// d2 v).  The factor 4 is common to every tap of a pixel and cancels in the normalisation by the sum of the weights.
+// The clamp min(d2, clp) is a packed 16-bit INTEGER min (VIMNMX.S16x2, integer pipe): clp > 0, so comparing the bit
+// patterns as signed integers orders every non-negative d2 correctly and returns d2 itself when rounding made it slightly
+// negative — identical to __hmin2 for finite inputs, off the pipe the HFMA2s use.
 __device__ __forceinline__ __half2 tap_weight_unclamped(__half2 d2, __half2 lob) {
-  const __half2 wb = __hfma2(__hfma2(h2c(0.25f), d2, h2c(-1.25f)), d2, h2c(1.0f));
-  __half2 wa = __hfma2(lob, d2, h2c(-1.0f));
-  wa = __hmul2(wa, wa);
-  return __hmul2(wb, wa);
+  const __half2 v = __hfma2(lob, d2, h2c(-1.0f));
+  const __half2 p = __hfma2(d2, v, __hneg2(v));
+  return __hmul2(p, __hfma2(v, h2c(-3.0f), p));
 }
 __device__ __forceinline__ __half2 tap_weight(__half2 d2, __half2 lob, __half2 clp) {
 #ifdef FSR1_CPU_EMU

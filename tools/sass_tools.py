@@ -2,6 +2,8 @@
 
   python tools/sass_tools.py hist [substring]      opcode histogram per kernel (largest basic blocks with --blocks)
   python tools/sass_tools.py snapshot FILE         save the instruction streams of every kernel
+  python tools/sass_tools.py loops BINARY          opcode histogram of each kernel's largest loop (the timed loop of
+                                                   tools/ubench_pipes.cu: one iteration)
   python tools/sass_tools.py diff FILE             compare the current library against a snapshot: lists kernels whose
                                                    instruction stream changed (used to prove that adding an opt-in
                                                    variant leaves every production kernel byte-for-byte the same)
@@ -17,8 +19,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "fidelityfx-fsr_b200", "lib", "libfsr1_b200.so")
 
 
-def kernels():
-    out = subprocess.run(["cuobjdump", "-sass", LIB], capture_output=True, text=True).stdout
+def kernels(path=LIB):
+    out = subprocess.run(["cuobjdump", "-sass", path], capture_output=True, text=True).stdout
     d, cur = {}, None
     for line in out.splitlines():
         m = re.search(r"Function : (\S+)", line)
@@ -66,6 +68,17 @@ def blocks(ins):
 
 def main():
     cmd = sys.argv[1] if len(sys.argv) > 1 else "hist"
+    if cmd == "loops":
+        for name, ins in kernels(sys.argv[2]).items():
+            body = []
+            for a, t in ins:  # the largest loop: from the target of a backward branch up to that branch
+                m = re.search(r"\bBRA\b.*?0x([0-9a-f]+)", t)
+                if m and int(m.group(1), 16) < a:
+                    loop = [(b, u) for b, u in ins if int(m.group(1), 16) <= b <= a]
+                    body = loop if len(loop) > len(body) else body
+            print("%-28s %4d SASS per iteration: %s" % (demangle(name), len(body),
+                                                         dict(collections.Counter(opcode(t) for _, t in body).most_common(6))))
+        return
     ks = kernels()
     if cmd == "hist":
         sub = [a for a in sys.argv[2:] if not a.startswith("--")]
